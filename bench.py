@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""Benchmark of the HAWQ integer forward path on B200 (contract in the task statement / DESIGN.md §Measurement).
+"""Benchmark of the HAWQ integer forward path on B200 (DESIGN.md §Measurement).
 
   python bench.py --gpus N --steps K --warmup W            one JSON line: images/s of the quantized ResNet forward
+  python bench.py ... --dump-outputs DIR                   also write the logits of the last timed step to DIR/logits.npy
   python bench.py --impl reference ...                     the reference's CPU path (oracle port) on the host cores
 
 A "step" = one forward of the frozen quantized ResNet over one batch of synthetic int8 images per GPU.
@@ -16,6 +17,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -24,6 +27,7 @@ import torch  # noqa: E402
 METRIC = "images/sec ResNet-50 W8A8 & W4A4 @batch128, 1/2/4/8xB200; % int-TC roofline"
 MACS_PER_IMAGE = {"resnet18": 1.8141e9, "resnet50": 3.8580e9, "resnet101": 7.57e9}
 INT8_TC_PEAK_OPS = 4.5e15        # nominal dense int8 tcgen05 peak (op/s); reported for context only
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def parse():
@@ -43,7 +47,27 @@ def parse():
     ap.add_argument("--a4-storage", default="byte", choices=["byte", "packed"],
                     help="HBM container of 4-bit activations: one value per byte (default, consumed directly by the int8 tensor-core kernels) or packed nibbles expanded on chip")
     ap.add_argument("--detail", default="", help="write per-layer timings to this JSON file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the logits of the last timed step to DIR/logits.npy (float32; inputs are seeded, so runs with the same "
+                         "arguments see the same images and two builds can be compared output for output)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
+    return a
+
+
+def dump_outputs(path, arrays):
+    """Write every array as <path>/<name>.npy in float32.  An array over DUMP_LIMIT_BYTES is replaced by a fixed sample of its rows
+    (seed 0, in row order), the same in every run."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.to("cpu", torch.float32).numpy()
+        if a.nbytes > DUMP_LIMIT_BYTES:
+            rows = DUMP_LIMIT_BYTES // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -270,11 +294,12 @@ def run_ours(a):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(a.steps):
-        step(i, dev_pool)
+        out = step(i, dev_pool)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     flag = int(eng.flag.item())
+    last = out.clone() if a.dump_outputs and rank == 0 else None     # later legs replay the same graph into the same buffer
     # ---- end-to-end through the public call with host buffers ("e2e")
     # public call: CompiledModel.run_pipelined(host batches) -> host logits; per step it copies the pinned int8 batch H2D,
     # replays the forward, reads logits + status flags back D2H (checked before the result is handed out)
@@ -350,6 +375,8 @@ def run_ours(a):
                            "frac_of_nominal": 2 * macs * value / INT8_TC_PEAK_OPS},
                 "parity": parity, "roofline": roof, "cpu_baseline": cpu, "batch8": small}
         print(json.dumps(line))
+        if last is not None:
+            dump_outputs(a.dump_outputs, {"logits": last})
         if a.detail and detail is not None:
             with open(a.detail, "w") as f:
                 json.dump(detail, f, indent=1)

@@ -7,6 +7,8 @@ Outputs (small, committed):
   net_<arch>_<scheme>.npz   whole-network: act ranges, per-QuantAct checksums of the activation integers,
                             per-layer checksums of weight_integer / bias_integer, logits  (batch 2)
   net_mobilenetv2_w1_<scheme>.npz   the same for MobileNetV2-1.0 (python tests/golden/make_golden.py --mobilenetv2 uniform8|uniform4)
+  ref_dropin.npz       the order in which the reference's graph code calls its quant modules, and an un-frozen MobileNetV2 output
+                       (python tests/golden/make_golden.py --dropin)
 Nothing here runs on the GPU box; tests only read the .npz files.
 """
 import hashlib
@@ -281,11 +283,42 @@ def make_kat_multibranch(ns):
     print("kat_multibranch ok")
 
 
+DROPIN_CONFIGS = [("resnet18", "uniform4"), ("resnet50", "bops_0.5"), ("mobilenetv2_w1", "uniform8")]
+
+
+def make_ref_dropin(ns):
+    """What tests/test_reference_dropin.py compares the reference's graph code against: the order in which the reference's
+    ResNet / MobileNetV2 graph code calls its quant modules in the un-frozen calibration forward, and the fp32 output of a second
+    un-frozen MobileNetV2 forward (the reference's own modules, ranges still moving)."""
+    from hawq_b200.synthetic import synthetic_float_mobilenetv2
+    from tests.util import QUANT_MODULES, quant_call_order
+    kinds = tuple(getattr(ns.quant_modules, n) for n in QUANT_MODULES)
+    out = {}
+    calib = synthetic_batch(CALIB_BATCH, CALIB_SEED)
+    for arch, scheme in DROPIN_CONFIGS:
+        if arch == "mobilenetv2_w1":
+            q = ns.q_mobilenetv2.q_mobilenetv2_w1(synthetic_float_mobilenetv2(0))
+        else:
+            q = {"resnet18": ns.q_resnet.q_resnet18, "resnet50": ns.q_resnet.q_resnet50}[arch](synthetic_float_resnet(arch, 0))
+        rh.stamp_like_quant_train(q, ns.bit_config_dict["bit_config_%s_%s" % (arch, scheme)])
+        q.eval()
+        order = quant_call_order(q, calib, kinds)
+        out["calls_%s_%s" % (arch, scheme)] = np.array(json.dumps(order))
+        if arch == "mobilenetv2_w1":
+            with torch.no_grad():
+                out["unfrozen_%s_%s" % (arch, scheme)] = q(synthetic_batch(PARITY_BATCH, PARITY_SEED)).numpy()
+    np.savez_compressed(os.path.join(HERE, "ref_dropin.npz"), **out)
+    print("ref_dropin ok", {k: v.shape for k, v in out.items()})
+
+
 if __name__ == "__main__":
     torch.set_num_threads(os.cpu_count())
     ns = rh.load()
     if len(sys.argv) == 2 and sys.argv[1] == "--multibranch":  # QuantAct on concatenated branches (quant_modules.py:275-286)
         make_kat_multibranch(ns)
+        sys.exit(0)
+    if len(sys.argv) == 2 and sys.argv[1] == "--dropin":      # reference graph code: quant-module call order, un-frozen output
+        make_ref_dropin(ns)
         sys.exit(0)
     if len(sys.argv) == 3 and sys.argv[1] == "--mobilenetv2":  # e.g. --mobilenetv2 uniform8
         make_net_mobilenetv2(ns, sys.argv[2])

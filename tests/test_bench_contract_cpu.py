@@ -32,3 +32,11 @@ def test_reference_arm_json_line():
 def test_reference_arm_other_ranks_are_silent():
     r = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_bad_arguments_are_refused(tmp_path):
+    """No timed step to divide by, and an output dump of the CPU arm (it runs other inputs than the GPU path): usage errors."""
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert r.returncode == 2 and "error" in r.stderr and r.stdout == "", (args, r.stderr[-500:])
+    assert not os.listdir(tmp_path)

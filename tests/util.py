@@ -24,6 +24,23 @@ def sha_i32(a):
     return hashlib.sha256(np.ascontiguousarray(np.asarray(a).astype(np.int32)).tobytes()).hexdigest()
 
 
+QUANT_MODULES = ("QuantAct", "QuantBnConv2d", "QuantConv2d", "QuantLinear", "QuantAveragePool2d")
+
+
+def quant_call_order(q, x, kinds):
+    """Names of the modules of `q` whose type is in `kinds`, in the order q's graph code calls them during one forward of x."""
+    order = []
+    hooks = [m.register_forward_pre_hook(lambda mod, inp, name=name: order.append(name))
+             for name, m in q.named_modules() if type(m) in kinds]
+    try:
+        with torch.no_grad():
+            q(x)
+    finally:
+        for h in hooks:
+            h.remove()
+    return order
+
+
 def golden_act_ranges(meta):
     return {k: (v["x_min"], v["x_max"]) for k, v in meta["acts"].items()}
 
